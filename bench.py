@@ -5,6 +5,7 @@ per-GPU batch 128, loss_type=h_loss, Adam lr 5e-4), one process per GPU.
   python bench.py --gpus 1 --steps K --warmup W                      # our CUDA path (default numeric mode: see --numeric)
   python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
   python bench.py --impl reference ...                               # the restated reference (oracle/) on the host CPU
+  python bench.py ... --dump-outputs DIR                             # also write the last timed step's outputs as DIR/*.npy
 
 A step = one full pass of the hot path over one batch: regressor forward (dropout on), h4p losses, DLT, fused warp +
 all six photometric diagnostics (the reference fetches them every step, homography_CNN_synthetic.py:345), backward of
@@ -30,10 +31,17 @@ FWD_FLOP_PER_PAIR = 2.5208e9
 TRAIN_FLOP_PER_PAIR = 7.525e9
 
 
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError("must be >= 1, got %d" % v)
+    return v
+
+
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=positive_int, default=20, help="number of timed train steps")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--numeric", default=os.environ.get("UDH_NUMERIC", "auto"), choices=["auto", "fp32", "bf16", "bf16x3"],
@@ -43,7 +51,40 @@ def parse():
     ap.add_argument("--dp-diag", default="", choices=["", "nocomm"], help="multi-GPU diagnosis only: 'nocomm' skips the gradient allreduce")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the short BASELINE configs[2]/[3] side measurements")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned on rank 0 (and a fixed sample of the updated "
+                         "weights) as DIR/<name>.npy; the inputs are seeded, so two builds can be compared output for output")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return a
+
+
+# Seeded sample of the updated flat parameters written by --dump-outputs: the full 137 MB buffer is too large to keep.
+PARAM_SAMPLE = 1 << 20
+
+
+def snapshot_outputs(out, params):
+    """Host copies of what one train step hands its caller: every public entry of the returned dict and a fixed seeded
+    sample of the updated parameters (about 13 MB in all at batch 128)."""
+    import numpy as np
+    import torch
+    snap = {}
+    for k, v in out.items():
+        if k.startswith("_"):
+            continue
+        a = v.detach().cpu().numpy() if isinstance(v, torch.Tensor) else np.asarray(v)
+        snap[k] = a.astype(np.float64 if a.dtype == np.float64 else np.float32)
+    idx = np.sort(np.random.default_rng(0).integers(0, params.numel(), PARAM_SAMPLE))
+    snap["params_sample"] = params[torch.from_numpy(idx).to(params.device)].cpu().numpy().astype(np.float32)
+    return snap
+
+
+def write_outputs(d, snap):
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    for k, a in snap.items():
+        np.save(os.path.join(d, k + ".npy"), a)
 
 
 def measured_peaks():
@@ -147,7 +188,7 @@ def run_reference(args):
     if rank != 0:
         return
     sample_b = 4
-    steps, warmup = max(1, args.steps), max(0, args.warmup)
+    steps, warmup = args.steps, max(0, args.warmup)
     val, ms, cores = cpu_oracle_pairs_per_s(sample_b, steps, warmup, args.loss_type)
     line = {
         "impl": "reference", "metric": METRIC, "value": val, "unit": "pairs/s", "n_gpus": args.gpus, "steps": steps, "warmup": warmup,
@@ -189,9 +230,14 @@ def run_ours(args):
         numeric = "bf16x3"       # the parity-certified tensor-core mode is the headline; single-pass bf16 is a labelled side number
     B = PER_GPU_BATCH
     eng = engine.HomographyEngine(B, numeric=numeric, seed=0, loss_type=args.loss_type, lr=5e-4, device=dev, process_group=pg, world_size=world)
+    # Training amplifies rounding: the gradient sums use fp32 atomics, whose order varies from run to run, and TF-Adam
+    # normalises near-zero gradients to steps of about lr, so two runs drift apart within a few steps.  The last timed step
+    # therefore starts again from the seeded initial state (restored outside the timed windows): its inputs are then the
+    # same in every run and its outputs (--dump-outputs) agree to rounding.
+    init_state = dict(params=eng.params.clone(), adam_m=eng.adam_m.clone(), adam_v=eng.adam_v.clone(), global_step=eng.global_step)
     nb = 3
     batches = [synthetic.make_batch(B, seed=1000 * rank + i, device=dev) for i in range(nb)]
-    W, K = max(3, args.warmup), max(1, args.steps)
+    W, K = max(3, args.warmup), args.steps
 
     def barrier():
         if world > 1:
@@ -204,16 +250,25 @@ def run_ours(args):
     for i in range(W):
         eng.train_step(batches[i % nb])
     barrier()
-    # ---- the timed region: exactly K steps, nothing else on the stream (no per-phase events) ----
+    # ---- the timed region: exactly K steps, nothing else on the stream (no per-phase events); two windows, K - 1 steps
+    # and the last one, with the restore of the initial state between them ----
     launches0 = _lib.lib.udh_launch_count()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    r0, r1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    for i in range(K):
+    for i in range(K - 1):
         eng.train_step(batches[i % nb])
+    r0.record()
+    eng.load_state_dict(init_state)
+    del init_state
+    r1.record()
+    out = eng.train_step(batches[(K - 1) % nb])
     e1.record()
     barrier()
-    ms_total = e0.elapsed_time(e1)
+    ms_total = e0.elapsed_time(r0) + r1.elapsed_time(e1)
     launches = _lib.lib.udh_launch_count() - launches0
+    # the step's results live in the engine's static buffers: copy them before the next step overwrites them
+    dumped = snapshot_outputs(out, eng.params) if args.dump_outputs and rank == 0 else None
     # ---- the same K steps again with the library's per-phase CUDA-event brackets (udh_prof_*): per-kernel durations for the
     # roofline.  Kept out of the headline region because ~80 event records per step serialise kernel boundaries. ----
     _lib.lib.udh_prof_enable(1); _lib.lib.udh_prof_reset()
@@ -362,6 +417,8 @@ def run_ours(args):
         "other_configs": extras,
     }
     print(json.dumps(line))
+    if dumped is not None:
+        write_outputs(args.dump_outputs, dumped)
     if world > 1:
         dist.destroy_process_group()
 
