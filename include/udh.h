@@ -251,29 +251,18 @@ int udh_warp_image_u8(const uint8_t* U, const float* H, uint8_t* out, int B, int
  * udh_prof_read synchronises on them and returns the accumulated device time and the number of brackets.
  * Must be off while a stream is being captured into a CUDA graph. */
 unsigned long long udh_launch_count(void);
-/* Leave n SMs free in the persistent one-CTA-per-SM tensor-core kernels (process-wide).  Used in data-parallel runs so
- * that the NCCL allreduce kernel overlapping the backward gets its own SMs instead of displacing persistent CTAs (a
- * displaced CTA would only start after another one finishes, i.e. serialise its whole share of the work). */
-int udh_set_sm_reserve(int n);
-/* Same, but only for the backward kernels of conv4_1 / conv4_2 (the launches that run while the fully connected gradients
- * are being all-reduced on the communication stream).  A persistent kernel with a static item schedule that finds n of its
- * SMs taken by the NCCL kernel runs those CTAs in a second wave (2x its time); with <= 2 items per CTA these four launches
- * lose nothing by starting on (SMs - n) CTAs, so reserving NCCL's CTA count here removes the collision. */
+/* Leave n SMs free in the persistent one-CTA-per-SM backward kernels of conv4_1 / conv4_2 (process-wide): the launches that
+ * run while the fully connected gradients are being all-reduced on the communication stream.  A persistent kernel with a
+ * static item schedule that finds n of its SMs taken by the NCCL kernel runs those CTAs in a second wave (2x its time); with
+ * <= 2 items per CTA these four launches lose nothing by starting on (SMs - n) CTAs, so reserving NCCL's CTA count here
+ * removes the collision. */
 int udh_set_sm_reserve_top(int n);
-/* CTAs (of 256 threads) of the Adam launches that follow; 0 = the default, enough to fill the device.  An update that runs
- * on a second stream underneath the conv backward is given one or two CTAs per SM so that the persistent tensor-core CTAs
- * (one per SM, ~200 KB of shared memory, <= 256 threads) stay co-resident with it instead of queueing behind it. */
-int udh_set_adam_grid(int blocks);
 /* A point inside the conv backward for a second stream to start at: with layer = 7..0 (conv4_2..conv1_1; -1 = off) every
  * conv backward that follows records an internal event on its stream right before the backward kernels of that layer, and
  * udh_bwd_marker_wait(stream) makes `stream` wait for the most recent record (no-op before the first).  The engine uses it
  * to run the fused gradient-reduce / Adam / weight-multicast kernel under the wide 64-channel layers' backward (tensor-bound)
  * rather than under conv4_x / conv3_x (short, latency-bound launches that a co-running streaming kernel slows 3-5x). */
 int udh_set_bwd_marker(int layer);
-/* SMs the persistent backward kernels of the marker layer and of the layers below it leave free (0 = none): a kernel of
- * 200+ KB of shared memory per CTA cannot share an SM with anything, so the second stream's kernel gets SMs of its own for
- * the length of that window and is launched with exactly that many CTAs. */
-int udh_set_sm_reserve_marker(int n);
 int udh_bwd_marker_wait(void* stream);
 
 /* Row G + the optimiser for ONE rank's shard of a replicated tensor, over NVSwitch multicast memory (csrc/dp_update.cu):

@@ -7,7 +7,7 @@ from ctypes import POINTER, c_char_p, c_double, c_float, c_int, c_int64, c_size_
 from . import build_ext
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = build_ext.lib_path()      # libudh.so (UDH_LIB_VARIANT selects an experimental build variant)
+LIB_PATH = build_ext.LIB
 
 OK, EINVAL, ECUDA, ENOSUP, EWS = 0, -1, -2, -3, -4
 NUMERIC_FP32, NUMERIC_BF16, NUMERIC_BF16X3 = 0, 1, 2
@@ -101,12 +101,9 @@ SIGNATURES = {
     "udh_synth_scene_u8": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_uint64, c_void_p]),
     "udh_warp_image_u8": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "udh_launch_count": (c_ulonglong, []),
-    "udh_set_sm_reserve": (c_int, [c_int]),
     "udh_set_sm_reserve_top": (c_int, [c_int]),
-    "udh_set_adam_grid": (c_int, [c_int]),
     "udh_crc32c": (c_uint32, [c_void_p, c_size_t, c_uint32]),
     "udh_set_bwd_marker": (c_int, [c_int]),
-    "udh_set_sm_reserve_marker": (c_int, [c_int]),
     "udh_bwd_marker_wait": (c_int, [c_void_p]),
     "udh_prof_enable": (c_int, [c_int]),
     "udh_prof_reset": (c_int, []),

@@ -1,12 +1,9 @@
 """Build libudh.so in-tree with nvcc for sm_100a (no torch in the link line: the library is a plain C ABI).
 
 Concurrency: several ranks (torchrun) may import the package at once on a fresh clone.  The build runs under an exclusive
-fcntl lock on `build/.lock`, compiles into a per-variant object directory, links to a temporary name and publishes the
-library with an atomic rename — a concurrent importer either waits for the lock and then finds the library up to date, or
-loads the previous complete file; it never sees a half-written one.
-
-Variants: UDH_LIB_VARIANT=<name> builds libudh_<name>.so with the extra nvcc flags VARIANTS[name] into its own object
-directory (used for A/B experiments on the GPU box; the product is the default variant and the only one listed).
+fcntl lock on `build/.lock`, compiles into `build/`, links to a temporary name and publishes the library with an atomic
+rename — a concurrent importer either waits for the lock and then finds the library up to date, or loads the previous
+complete file; it never sees a half-written one.
 """
 import fcntl
 import glob
@@ -17,22 +14,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 
-VARIANTS = {"": []}
-
-
-def variant():
-    v = os.environ.get("UDH_LIB_VARIANT", "")
-    if v not in VARIANTS:
-        raise RuntimeError("unknown UDH_LIB_VARIANT %r (known: %s)" % (v, sorted(VARIANTS)))
-    return v
-
-
-def lib_path(v=None):
-    v = variant() if v is None else v
-    return os.path.join(HERE, "libudh%s.so" % ("_" + v if v else ""))
-
-
-LIB = lib_path("")
+LIB = os.path.join(HERE, "libudh.so")
 
 NVCC_FLAGS = [
     "-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
@@ -44,33 +26,30 @@ def sources():
     return sorted(glob.glob(os.path.join(CSRC, "*.cu")))
 
 
-def needs_build(v=None):
-    lib = lib_path(v)
-    if not os.path.exists(lib):
+def needs_build():
+    if not os.path.exists(LIB):
         return True
-    t = os.path.getmtime(lib)
+    t = os.path.getmtime(LIB)
     deps = sources() + glob.glob(os.path.join(CSRC, "*.cuh")) + [os.path.join(HERE, "..", "include", "udh.h")]
     return any(os.path.getmtime(d) > t for d in deps)
 
 
-def build(force=False, verbose=False, v=None):
-    v = variant() if v is None else v
-    lib = lib_path(v)
-    if not force and not needs_build(v):
-        return lib
-    bdir = os.path.join(HERE, "build" + ("_" + v if v else ""))
+def build(force=False, verbose=False):
+    if not force and not needs_build():
+        return LIB
+    bdir = os.path.join(HERE, "build")
     os.makedirs(bdir, exist_ok=True)
     with open(os.path.join(bdir, ".lock"), "w") as lock:
         fcntl.flock(lock, fcntl.LOCK_EX)
         try:
-            if not force and not needs_build(v):        # another process built it while we waited for the lock
-                return lib
+            if not force and not needs_build():         # another process built it while we waited for the lock
+                return LIB
             nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
             objs, procs = [], []
             for src in sources():
                 obj = os.path.join(bdir, os.path.basename(src)[:-3] + ".o")
                 objs.append(obj)
-                cmd = [nvcc] + NVCC_FLAGS + VARIANTS[v] + (["-Xptxas", "-v"] if verbose else []) + ["-c", src, "-o", obj]
+                cmd = [nvcc] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-c", src, "-o", obj]
                 procs.append((src, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)))
             ok = True
             for src, p in procs:
@@ -79,13 +58,13 @@ def build(force=False, verbose=False, v=None):
                     sys.stderr.write("== %s\n%s\n" % (os.path.basename(src), out))
                 ok = ok and p.returncode == 0
             if not ok:
-                raise RuntimeError("nvcc failed building %s" % os.path.basename(lib))
-            tmp = "%s.tmp.%d" % (lib, os.getpid())
+                raise RuntimeError("nvcc failed building %s" % os.path.basename(LIB))
+            tmp = "%s.tmp.%d" % (LIB, os.getpid())
             subprocess.check_call([nvcc, "-shared", "-o", tmp] + objs + ["-gencode", "arch=compute_100a,code=sm_100a"])
-            os.replace(tmp, lib)                        # atomic publish
+            os.replace(tmp, LIB)                        # atomic publish
         finally:
             fcntl.flock(lock, fcntl.LOCK_UN)
-    return lib
+    return LIB
 
 
 PROBE_LIB = os.path.join(HERE, "libudh_probe.so")

@@ -21,7 +21,7 @@ enum ProfTag {
   PROF_H4P_LOSS, PROF_ADAM, PROF_ELTWISE, PROF_TC_PREP, PROF_NUM_TAGS
 };
 extern unsigned long long g_launches;
-extern int g_sm_reserve;      // SMs the persistent tensor-core kernels leave free (udh_set_sm_reserve)
+extern int g_sm_reserve;      // SMs the persistent tensor-core kernels leave free (set per layer by the backward loops)
 extern int g_sm_reserve_top;  // SMs the conv4_x backward kernels leave free (udh_set_sm_reserve_top): these few launches run
                               // while the fc-gradient allreduce occupies SMs; they have <= 2 items per CTA either way
 // CTAs a persistent one-CTA-per-SM kernel should launch on the current device
@@ -32,14 +32,9 @@ inline int persistent_ctas() {
   const int n = sms - g_sm_reserve;
   return n > 0 ? n : 1;
 }
-extern int g_bwd_marker_layer, g_sm_reserve_marker;   // udh_set_bwd_marker / udh_set_sm_reserve_marker
-// SMs the persistent backward kernels of conv layer i leave free: the global reserve, conv4_x's (udh_set_sm_reserve_top), and
-// from the marker layer down the SMs handed to the second stream's kernel (udh_set_sm_reserve_marker)
-inline int bwd_sm_reserve(int i, int reserve_all) {
-  int r = (i >= 6 && g_sm_reserve_top > reserve_all) ? g_sm_reserve_top : reserve_all;
-  if (g_bwd_marker_layer >= 0 && i <= g_bwd_marker_layer && g_sm_reserve_marker > r) r = g_sm_reserve_marker;
-  return r;
-}
+extern int g_bwd_marker_layer;   // udh_set_bwd_marker
+// SMs the persistent backward kernels of conv layer i leave free: conv4_x's reserve (udh_set_sm_reserve_top), none elsewhere
+inline int bwd_sm_reserve(int i) { return i >= 6 ? g_sm_reserve_top : 0; }
 int bwd_marker_record(int layer, cudaStream_t st);   // udh_set_bwd_marker: event before layer's backward kernels
 void prof_begin(int tag, cudaStream_t st);
 void prof_end(int tag, cudaStream_t st);

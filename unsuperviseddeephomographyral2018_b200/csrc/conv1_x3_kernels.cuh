@@ -12,7 +12,6 @@
 namespace udh {
 namespace tc {
 
-template <int FMT>
 __device__ __forceinline__ void build_im2col_row_x3(uint8_t* tile, int r, const float* __restrict__ I1, const float* __restrict__ I2,
                                                     int n, int y, int x, int H, int W, bool ones_col) {
   float v[24];
@@ -38,7 +37,7 @@ __device__ __forceinline__ void build_im2col_row_x3(uint8_t* tile, int r, const 
   for (int c = 0; c < 3; ++c) {
     uint32_t hi[4], lo[4];
 #pragma unroll
-    for (int h = 0; h < 4; ++h) split2<FMT>(v[c * 8 + 2 * h], v[c * 8 + 2 * h + 1], hi[h], lo[h]);
+    for (int h = 0; h < 4; ++h) split2(v[c * 8 + 2 * h], v[c * 8 + 2 * h + 1], hi[h], lo[h]);
     asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(rowaddr + (uint32_t)((c ^ (r & 7)) << 4)), "r"(hi[0]), "r"(hi[1]),
                  "r"(hi[2]), "r"(hi[3]) : "memory");
     asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(rowaddr + (uint32_t)(((4 + c) ^ (r & 7)) << 4)), "r"(lo[0]), "r"(lo[1]),
@@ -48,8 +47,7 @@ __device__ __forceinline__ void build_im2col_row_x3(uint8_t* tile, int r, const 
 
 // ------------------------------------------------------------------------------------------------------------- forward
 constexpr int kConv1X3CtasPerSm = 3;
-template <int FMT>
-__global__ void __launch_bounds__(160, kConv1X3CtasPerSm)
+static __global__ void __launch_bounds__(160, kConv1X3CtasPerSm)
 conv1_x3_fwd_kernel(const __grid_constant__ CUtensorMap tmOut, const Conv1Geom g, const float* __restrict__ I1,
                     const float* __restrict__ I2, const float* __restrict__ w, const float* __restrict__ bias,
                     uint32_t* __restrict__ mask_out) {
@@ -79,7 +77,7 @@ conv1_x3_fwd_kernel(const __grid_constant__ CUtensorMap tmOut, const Conv1Geom g
       const float f0 = kk < 18 ? __ldg(w + kk * 64 + co) : (kk == 18 ? __ldg(bias + co) : 0.f);
       const float f1 = kk + 1 < 18 ? __ldg(w + (kk + 1) * 64 + co) : (kk + 1 == 18 ? __ldg(bias + co) : 0.f);
       uint32_t hi, lo;
-      split2<FMT>(f0, f1, hi, lo);
+      split2(f0, f1, hi, lo);
       p1[h] = hi;
       p2[h] = c < 4 ? lo : 0u;
     }
@@ -116,7 +114,7 @@ conv1_x3_fwd_kernel(const __grid_constant__ CUtensorMap tmOut, const Conv1Geom g
         const int n = row / g.H, y = row - n * g.H;
         const int b = i & 1;
         mbar_wait(&a_empty[b], ((i >> 1) & 1) ^ 1);
-        build_im2col_row_x3<FMT>(sA + b * 16384, px, I1, I2, n, y, seg * 128 + px, g.H, g.W, true);
+        build_im2col_row_x3(sA + b * 16384, px, I1, I2, n, y, seg * 128 + px, g.H, g.W, true);
         fence_proxy_async();
         mbar_arrive(&a_full[b]);
       }
@@ -145,7 +143,7 @@ conv1_x3_fwd_kernel(const __grid_constant__ CUtensorMap tmOut, const Conv1Geom g
           }
           mo[c] = mw;
 #pragma unroll
-          for (int k = 0; k < 16; ++k) split2<FMT>(v[2 * k], v[2 * k + 1], hi[c][k], lo[c][k]);
+          for (int k = 0; k < 16; ++k) split2(v[2 * k], v[2 * k + 1], hi[c][k], lo[c][k]);
         }
         tc_fence_before();
         mbar_arrive(&t_empty[b]);
@@ -173,7 +171,7 @@ conv1_x3_fwd_kernel(const __grid_constant__ CUtensorMap tmOut, const Conv1Geom g
     __syncwarp();
   } else {
     // ---- MMA issuer (whole warp converged)
-    constexpr uint32_t idesc = make_idesc_f16kind(128, 64, 0, 0, FMT, FMT);
+    constexpr uint32_t idesc = make_idesc_bf16(128, 64, 0, 0);
     const uint32_t w1_lo = desc_lo(smem_u32(sW), 16), w2_lo = desc_lo(smem_u32(sW + 8192), 16);
     for (int i = 0; i < my_tiles; ++i) {
       const int b = i & 1;
@@ -202,8 +200,7 @@ conv1_x3_fwd_kernel(const __grid_constant__ CUtensorMap tmOut, const Conv1Geom g
 
 // ------------------------------------------------------------------------------------------------------------- wgrad
 constexpr int kConv1X3WgradCtasPerSm = 2;
-template <int FMT_X, int FMT_G>
-__global__ void __launch_bounds__(160, kConv1X3WgradCtasPerSm)
+static __global__ void __launch_bounds__(160, kConv1X3WgradCtasPerSm)
 conv1_x3_wgrad_kernel(const __grid_constant__ CUtensorMap tmG, const Conv1Geom g, const float* __restrict__ I1,
                       const float* __restrict__ I2, float* __restrict__ dW, float* __restrict__ db) {
   extern __shared__ uint8_t raw[];
@@ -244,7 +241,7 @@ conv1_x3_wgrad_kernel(const __grid_constant__ CUtensorMap tmG, const Conv1Geom g
       const int n = row / g.H, y = row - n * g.H;
       const int b = i & 1;
       mbar_wait(&empty[b], ((i >> 1) & 1) ^ 1);
-      build_im2col_row_x3<FMT_X>(sA + b * 16384, px, I1, I2, n, y, seg * 128 + px, g.H, g.W, true);
+      build_im2col_row_x3(sA + b * 16384, px, I1, I2, n, y, seg * 128 + px, g.H, g.W, true);
       fence_proxy_async();
       mbar_arrive(&a_full[b]);
     }
@@ -267,7 +264,7 @@ conv1_x3_wgrad_kernel(const __grid_constant__ CUtensorMap tmG, const Conv1Geom g
       }
     }
   } else {
-    constexpr uint32_t idesc = make_idesc_f16kind(64, 64, 1, 1, FMT_X, FMT_G);
+    constexpr uint32_t idesc = make_idesc_bf16(64, 64, 1, 1);
     for (int i = 0; i < my_tiles; ++i) {
       const int tile = (int)blockIdx.x + i * (int)gridDim.x;
       const int seg = tile % segs, row = tile / segs;

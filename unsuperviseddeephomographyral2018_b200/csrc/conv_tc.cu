@@ -507,13 +507,12 @@ int tc_cnn_bwd_convs(const float* params, const size_t* poff, const float* I1, c
     ProfScope ps(PROF_TC_PREP, st);        // (the mirrored weight packs were made by the forward of this step)
     TRY(pad_cast(gA, Gb(7), B, P / 8, P / 8, 128, st));
   }
-  const int reserve_all = g_sm_reserve;
-  struct RestoreReserve { int v; ~RestoreReserve() { g_sm_reserve = v; } } restore_reserve{reserve_all};
+  struct RestoreReserve { ~RestoreReserve() { g_sm_reserve = 0; } } restore_reserve;   // outside the conv backward every SM is used
   for (int i = 7; i >= 0; --i) {
     TRY(bwd_marker_record(i, st));
     const int s = P / kConv[i].div;
     const int cin = kConv[i].cin, cout = kConv[i].cout;
-    g_sm_reserve = bwd_sm_reserve(i, reserve_all);   // see udh_set_sm_reserve_top / udh_set_sm_reserve_marker
+    g_sm_reserve = bwd_sm_reserve(i);   // see udh_set_sm_reserve_top
     {
       ProfScope ps(PROF_CONV_WGRAD0 + i, st);
       if (i == 0) {

@@ -12,7 +12,6 @@
 #include "gemm_tc_kernels.cuh"
 #include "conv1_x3_kernels.cuh"
 #include "tc_layout.cuh"
-#include "x3_config.cuh"
 
 namespace udh {
 
@@ -21,12 +20,9 @@ namespace {
 using namespace tcl;
 #define TRY UDH_TRY
 
-constexpr int kFwd = kX3Fwd, kGrad = kX3Grad;     // limb formats (x3_config.cuh)
-
-template <int FMT>
 __device__ __forceinline__ void split1(float v, uint16_t& hi, uint16_t& lo) {
   uint32_t h, l;
-  tc::split2<FMT>(v, 0.f, h, l);
+  tc::split2(v, 0.f, h, l);
   hi = (uint16_t)(h & 0xFFFFu); lo = (uint16_t)(l & 0xFFFFu);
 }
 
@@ -50,7 +46,7 @@ __global__ void pack_all_weights_x3_kernel(PackTableX3 t) {
     const int kc = cb * 64 + k;
     const float v = dgrad ? w[((size_t)(8 - tap) * Cin + n) * Cout + kc] : w[((size_t)tap * Cin + kc) * Cout + n];
     uint16_t hi, lo;
-    if (dgrad) split1<kGrad>(v, hi, lo); else split1<kFwd>(v, hi, lo);
+    split1(v, hi, lo);
     const size_t blk = (size_t)(tap * CBk + cb) * 2;
     dst[(blk * N + n) * 64 + k] = hi;
     dst[((blk + 1) * N + n) * 64 + k] = lo;
@@ -58,7 +54,6 @@ __global__ void pack_all_weights_x3_kernel(PackTableX3 t) {
 }
 
 // fp32 [B,H,W,C] -> limb stream [B,H+2,W+2,2C] interior (borders untouched = zero)
-template <int FMT>
 __global__ void pad_cast_x3_kernel(const float* __restrict__ src, uint16_t* __restrict__ dst, int B, int H, int W, int C) {
   pdl_wait(); pdl_trigger();
   const int C4 = C >> 2;
@@ -71,8 +66,8 @@ __global__ void pad_cast_x3_kernel(const float* __restrict__ src, uint16_t* __re
     const int n = r / H;
     const float4 v = __ldg(reinterpret_cast<const float4*>(src) + i);
     uint2 hi, lo;
-    tc::split2<FMT>(v.x, v.y, hi.x, lo.x);
-    tc::split2<FMT>(v.z, v.w, hi.y, lo.y);
+    tc::split2(v.x, v.y, hi.x, lo.x);
+    tc::split2(v.z, v.w, hi.y, lo.y);
     uint16_t* p = dst + (((size_t)n * (H + 2) + y + 1) * (W + 2) + x + 1) * (2 * C) + c4 * 4;
     *reinterpret_cast<uint2*>(p) = hi;
     *reinterpret_cast<uint2*>(p + C) = lo;
@@ -80,7 +75,6 @@ __global__ void pad_cast_x3_kernel(const float* __restrict__ src, uint16_t* __re
 }
 
 // limb stream interior -> fp32 [B,H,W,C] (debug / tests)
-template <int FMT>
 __global__ void unpad_cast_x3_kernel(const uint16_t* __restrict__ src, float* __restrict__ dst, int B, int H, int W, int C) {
   const int C4 = C >> 2;
   const size_t total = (size_t)B * H * W * C4;
@@ -92,13 +86,12 @@ __global__ void unpad_cast_x3_kernel(const uint16_t* __restrict__ src, float* __
     const int n = r / H;
     const uint16_t* p = src + (((size_t)n * (H + 2) + y + 1) * (W + 2) + x + 1) * (2 * C) + c4 * 4;
     const uint2 hi = __ldg(reinterpret_cast<const uint2*>(p)), lo = __ldg(reinterpret_cast<const uint2*>(p + C));
-    const float2 a = tc::join2<FMT>(hi.x, lo.x), b = tc::join2<FMT>(hi.y, lo.y);
+    const float2 a = tc::join2(hi.x, lo.x), b = tc::join2(hi.y, lo.y);
     reinterpret_cast<float4*>(dst)[i] = make_float4(a.x, a.y, b.x, b.y);
   }
 }
 
 // fp32 [rows][cols] -> [rows][hi(cols) | lo(cols)]
-template <int FMT>
 __global__ void cast_x3_kernel(const float* __restrict__ src, uint16_t* __restrict__ dst, size_t rows, int cols) {
   pdl_wait(); pdl_trigger();
   const int C4 = cols >> 2;
@@ -108,8 +101,8 @@ __global__ void cast_x3_kernel(const float* __restrict__ src, uint16_t* __restri
     const int c4 = (int)(i - r * C4);
     const float4 v = __ldg(reinterpret_cast<const float4*>(src) + i);
     uint2 hi, lo;
-    tc::split2<FMT>(v.x, v.y, hi.x, lo.x);
-    tc::split2<FMT>(v.z, v.w, hi.y, lo.y);
+    tc::split2(v.x, v.y, hi.x, lo.x);
+    tc::split2(v.z, v.w, hi.y, lo.y);
     uint16_t* p = dst + r * (size_t)(2 * cols) + c4 * 4;
     *reinterpret_cast<uint2*>(p) = hi;
     *reinterpret_cast<uint2*>(p + cols) = lo;
@@ -117,29 +110,26 @@ __global__ void cast_x3_kernel(const float* __restrict__ src, uint16_t* __restri
 }
 
 // fp32 [n] -> hi[n], lo[n] (fc1's weight mirror: W_hi rows then W_lo rows)
-template <int FMT>
 __global__ void cast_planes_x3_kernel(const float* __restrict__ src, uint16_t* __restrict__ hi_dst, uint16_t* __restrict__ lo_dst, size_t n4) {
   pdl_wait(); pdl_trigger();
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (size_t)gridDim.x * blockDim.x) {
     const float4 v = __ldg(reinterpret_cast<const float4*>(src) + i);
     uint2 hi, lo;
-    tc::split2<FMT>(v.x, v.y, hi.x, lo.x);
-    tc::split2<FMT>(v.z, v.w, hi.y, lo.y);
+    tc::split2(v.x, v.y, hi.x, lo.x);
+    tc::split2(v.z, v.w, hi.y, lo.y);
     reinterpret_cast<uint2*>(hi_dst)[i] = hi;
     reinterpret_cast<uint2*>(lo_dst)[i] = lo;
   }
 }
 
-template <int FMT>
 __device__ __forceinline__ void join8(const uint4& h, const uint4& l, float (&f)[8]) {
-  const float2 a = tc::join2<FMT>(h.x, l.x), b = tc::join2<FMT>(h.y, l.y), c = tc::join2<FMT>(h.z, l.z), d = tc::join2<FMT>(h.w, l.w);
+  const float2 a = tc::join2(h.x, l.x), b = tc::join2(h.y, l.y), c = tc::join2(h.z, l.z), d = tc::join2(h.w, l.w);
   f[0] = a.x; f[1] = a.y; f[2] = b.x; f[3] = b.y; f[4] = c.x; f[5] = c.y; f[6] = d.x; f[7] = d.y;
 }
 __device__ __forceinline__ uint16_t half_of(uint32_t w, int odd) { return (uint16_t)(odd ? (w >> 16) : (w & 0xFFFFu)); }
 
 // 2x2/2 max pool on limb streams.  The decision uses the value hi + lo; the winner's limbs are copied unchanged, so pooling
 // adds no rounding.  Routing codes as in pool_fwd_bf16_kernel (3 bits per channel, 4 = maximum not positive).
-template <int FMT>
 __global__ void pool_fwd_x3_kernel(const uint16_t* __restrict__ in, uint16_t* __restrict__ out, uint32_t* __restrict__ codes,
                                    int B, int H, int W, int C) {
   pdl_wait(); pdl_trigger();
@@ -161,7 +151,7 @@ __global__ void pool_fwd_x3_kernel(const uint16_t* __restrict__ in, uint16_t* __
     h[3] = __ldg(reinterpret_cast<const uint4*>(p + rowp + pix));  l[3] = __ldg(reinterpret_cast<const uint4*>(p + rowp + pix + C));
     float f[4][8];
 #pragma unroll
-    for (int k = 0; k < 4; ++k) join8<FMT>(h[k], l[k], f[k]);
+    for (int k = 0; k < 4; ++k) join8(h[k], l[k], f[k]);
     uint32_t code = 0;
     uint32_t oh[4] = {0, 0, 0, 0}, ol[4] = {0, 0, 0, 0};
 #pragma unroll
@@ -228,11 +218,11 @@ __global__ void pool_bwd_x3_kernel(const uint32_t* __restrict__ codes, const uin
 }
 
 // ---------------------------------------------------------------------------------------------------- launchers
-template <int N_OUT, int CB, int T, int FA, int FW, int FO, bool WIDE, int STAGES>
+template <int N_OUT, int CB, int T, bool WIDE, int STAGES>
 int launch_conv_x3_impl(const CUtensorMap& tmA128, const CUtensorMap& tmAhh, const CUtensorMap& tmW, const CUtensorMap& tmOut, const tc::ConvGeom& g,
                         int stages, size_t smem, const float* bias, const uint32_t* mask_bits, uint32_t* mask_out, float* out_f32, int relu,
                         float out_scale, cudaStream_t st) {
-  auto kern = tc::tc_conv_x3_kernel<N_OUT, CB, T, FA, FW, FO, WIDE, STAGES>;
+  auto kern = tc::tc_conv_x3_kernel<N_OUT, CB, T, WIDE, STAGES>;
   UDH_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int sms = persistent_ctas();
   const int grid = g.num_items < sms ? g.num_items : sms;
@@ -240,7 +230,7 @@ int launch_conv_x3_impl(const CUtensorMap& tmA128, const CUtensorMap& tmAhh, con
   return check_launch("tc_conv_x3_kernel");
 }
 
-template <int N_OUT, int CB, int T, int FA, int FW, int FO, bool WIDE = false>
+template <int N_OUT, int CB, int T, bool WIDE = false>
 int launch_conv_x3(const uint16_t* x, const uint16_t* wpk, const float* bias, const uint32_t* mask_bits, uint32_t* mask_out,
                    uint16_t* out_limbs, float* out_f32, int relu, int B, int H, int W, float out_scale, cudaStream_t st) {
   tc::ConvGeom g;
@@ -264,29 +254,23 @@ int launch_conv_x3(const uint16_t* x, const uint16_t* wpk, const float* bias, co
   TRY(tc::make_tmap_bf16(&tmOut, out_limbs, 2, dimsO, strO, boxO));
   using S = tc::ConvX3Smem<N_OUT, CB, T, WIDE>;
   int stages = S::stages(g.abuf_rows);
-  UDH_REQUIRE(stages >= 2, "tc conv x3: activation rows (%d x %d blocks) leave no room for the weight ring", g.abuf_rows, 2 * CB);
-  // static ring (unrolled issue loop) when a depth of 6 or 3 fits: both divide the 18*CB (WIDE) / 27*CB stages of an item
-  // (measured: the 128-channel / CB = 2 instances are better off with the deeper runtime ring, so only WIDE uses it)
-  static const int static_env = [] { const char* e = getenv("UDH_X3_STATIC_RING"); return (e && e[0] == '0') ? 0 : 1; }();
-  const int use_static = WIDE ? static_env : 0;
-  constexpr int kSPI = (WIDE ? 18 : 27) * CB;
-  if constexpr (kSPI % 6 == 0) if (use_static && stages >= 6) {
-    stages = 6;
-    return launch_conv_x3_impl<N_OUT, CB, T, FA, FW, FO, WIDE, 6>(tmA128, tmAhh, tmW, tmOut, g, stages, S::fixed_bytes(g.abuf_rows) + (size_t)stages * S::kWStageBytes,
-                                                                  bias, mask_bits, mask_out, out_f32, relu, out_scale, st);
+  // WIDE: static ring (unrolled issue loop) of depth 6 when it fits, else 3 (both divide the 18 stages of an item; at W = 64
+  // six fit, at W = 128 four).  The other instances are better off with the deepest runtime ring that fits (measured).
+  UDH_REQUIRE(stages >= (WIDE ? 3 : 2), "tc conv x3: activation rows (%d x %d blocks) leave no room for the weight ring", g.abuf_rows, 2 * CB);
+  if constexpr (WIDE) stages = stages >= 6 ? 6 : 3;
+  const size_t smem = S::fixed_bytes(g.abuf_rows) + (size_t)stages * S::kWStageBytes;
+  if constexpr (WIDE) {
+    if (stages == 6)
+      return launch_conv_x3_impl<N_OUT, CB, T, true, 6>(tmA128, tmAhh, tmW, tmOut, g, stages, smem, bias, mask_bits, mask_out, out_f32, relu, out_scale, st);
+    return launch_conv_x3_impl<N_OUT, CB, T, true, 3>(tmA128, tmAhh, tmW, tmOut, g, stages, smem, bias, mask_bits, mask_out, out_f32, relu, out_scale, st);
+  } else {
+    return launch_conv_x3_impl<N_OUT, CB, T, false, 0>(tmA128, tmAhh, tmW, tmOut, g, stages, smem, bias, mask_bits, mask_out, out_f32, relu, out_scale, st);
   }
-  if (use_static && stages >= 3) {
-    stages = 3;
-    return launch_conv_x3_impl<N_OUT, CB, T, FA, FW, FO, WIDE, 3>(tmA128, tmAhh, tmW, tmOut, g, stages, S::fixed_bytes(g.abuf_rows) + (size_t)stages * S::kWStageBytes,
-                                                                  bias, mask_bits, mask_out, out_f32, relu, out_scale, st);
-  }
-  return launch_conv_x3_impl<N_OUT, CB, T, FA, FW, FO, WIDE, 0>(tmA128, tmAhh, tmW, tmOut, g, stages, S::fixed_bytes(g.abuf_rows) + (size_t)stages * S::kWStageBytes,
-                                                                bias, mask_bits, mask_out, out_f32, relu, out_scale, st);
 }
 
 // conv1_2 on row tiles (64 -> 64 channels, 128-wide images): ROWS = 1 forward fused with pool1 (writes the pooled two-limb
 // stream + routing codes), ROWS = 2 the dgrad (ordinary epilogue).  See conv_x3_kernels.cuh.
-template <int ROWS, int FA, int FW, int FO>
+template <int ROWS>
 int launch_conv_x3_rows(const uint16_t* x, const uint16_t* wpk, const float* bias, const uint32_t* mask_bits, uint32_t* codes_or_mask,
                         uint16_t* out_limbs, int relu, int B, int H, int W, cudaStream_t st) {
   UDH_REQUIRE(W == 128 && H % 2 == 0 && out_limbs, "tc conv x3 rows: needs W == 128, an even height and an output stream");
@@ -311,7 +295,7 @@ int launch_conv_x3_rows(const uint16_t* x, const uint16_t* wpk, const float* bia
   constexpr int kStages = 3;
   const size_t smem = S::fixed_bytes(g.abuf_rows) + (size_t)kStages * S::kWStageBytes;
   UDH_REQUIRE(smem <= 232448, "tc conv x3 rows: %zu bytes of shared memory exceed the 227 KiB limit", smem);
-  auto kern = tc::tc_conv_x3_kernel<64, 1, 2, FA, FW, FO, true, kStages, ROWS>;
+  auto kern = tc::tc_conv_x3_kernel<64, 1, 2, true, kStages, ROWS>;
   UDH_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int sms = persistent_ctas();
   const int grid = g.num_items < sms ? g.num_items : sms;
@@ -321,17 +305,13 @@ int launch_conv_x3_rows(const uint16_t* x, const uint16_t* wpk, const float* bia
   return check_launch("tc_conv_x3_kernel(rows)");
 }
 
-// one 3x3 conv on limb streams; (cin -> cout, image width) selects the kernel instance.  FA/FW/FO: limb formats.
-template <int FA, int FW, int FO>
+// one 3x3 conv on limb streams; (cin -> cout) selects the kernel instance
 int tc_conv_x3(const uint16_t* x, const uint16_t* wpk, const float* bias, const uint32_t* mask_bits, uint32_t* mask_out,
                uint16_t* out_limbs, float* out_f32, int relu, int B, int H, int W, int cin, int cout, cudaStream_t st) {
-  static const int wide = [] { const char* e = getenv("UDH_X3_WIDE"); return (e && e[0] == '0') ? 0 : 1; }();
-  if (cin == 64 && cout == 64 && wide) return launch_conv_x3<64, 1, 2, FA, FW, FO, true>(x, wpk, bias, mask_bits, mask_out, out_limbs, out_f32, relu, B, H, W, 1.0f, st);
-  if (cin == 64 && cout == 64 && W >= 128) return launch_conv_x3<64, 1, 3, FA, FW, FO>(x, wpk, bias, mask_bits, mask_out, out_limbs, out_f32, relu, B, H, W, 1.0f, st);
-  if (cin == 64 && cout == 64) return launch_conv_x3<64, 1, 4, FA, FW, FO>(x, wpk, bias, mask_bits, mask_out, out_limbs, out_f32, relu, B, H, W, 1.0f, st);
-  if (cin == 64 && cout == 128) return launch_conv_x3<128, 1, 2, FA, FW, FO>(x, wpk, bias, mask_bits, mask_out, out_limbs, out_f32, relu, B, H, W, 1.0f, st);
-  if (cin == 128 && cout == 64) return launch_conv_x3<64, 2, 2, FA, FW, FO>(x, wpk, bias, mask_bits, mask_out, out_limbs, out_f32, relu, B, H, W, 1.0f, st);
-  if (cin == 128 && cout == 128) return launch_conv_x3<128, 2, 2, FA, FW, FO>(x, wpk, bias, mask_bits, mask_out, out_limbs, out_f32, relu, B, H, W, 1.0f, st);
+  if (cin == 64 && cout == 64) return launch_conv_x3<64, 1, 2, true>(x, wpk, bias, mask_bits, mask_out, out_limbs, out_f32, relu, B, H, W, 1.0f, st);
+  if (cin == 64 && cout == 128) return launch_conv_x3<128, 1, 2>(x, wpk, bias, mask_bits, mask_out, out_limbs, out_f32, relu, B, H, W, 1.0f, st);
+  if (cin == 128 && cout == 64) return launch_conv_x3<64, 2, 2>(x, wpk, bias, mask_bits, mask_out, out_limbs, out_f32, relu, B, H, W, 1.0f, st);
+  if (cin == 128 && cout == 128) return launch_conv_x3<128, 2, 2>(x, wpk, bias, mask_bits, mask_out, out_limbs, out_f32, relu, B, H, W, 1.0f, st);
   set_error("tc_conv_x3: unsupported channel combination %d -> %d", cin, cout);
   return UDH_ENOSUP;
 }
@@ -366,7 +346,7 @@ int launch_wgrad_x3(const uint16_t* x, const uint16_t* gsrc, float* dW, float* d
   TRY(tc::make_tmap_bf16(&tmG, gsrc, 2, dimsG, strG, box128));
   const size_t smem = 1024 + 2 * ((size_t)CBX * g.xrows * 128 + (size_t)CBO * T * 16384) + 2 * tc::kConstBlockBytes + 256;
   UDH_REQUIRE(smem <= 232448, "tc wgrad x3: %zu bytes of shared memory exceed the 227 KiB limit", smem);
-  auto kern = tc::tc_wgrad_x3_kernel<N_OUT, CBX, T, kFwd, kGrad>;
+  auto kern = tc::tc_wgrad_x3_kernel<N_OUT, CBX, T>;
   UDH_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   launch_chain(kern, dim3(g.slice_cta[g.num_slices]), dim3(256), smem, st, tmX128, tmXhh, tmG, g, dW, db);
   return check_launch("tc_wgrad_x3_kernel");
@@ -389,7 +369,7 @@ int launch_wgrad64_x3(const uint16_t* x, const uint16_t* gsrc, float* dW, float*
   TRY(tc::make_tmap_bf16(&tmG136, gsrc, 2, dims, str, box136));
   const size_t smem = 1024 + 2 * ((size_t)g.xrows * 128 + (size_t)(T * 128 + 16) * 128) + 2 * tc::kConstBlockBytes + 256;
   UDH_REQUIRE(smem <= 232448, "tc wgrad64 x3: %zu bytes of shared memory exceed the 227 KiB limit", smem);
-  auto kern = tc::tc_wgrad64_x3_kernel<T, kFwd, kGrad>;
+  auto kern = tc::tc_wgrad64_x3_kernel<T>;
   UDH_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int sms = persistent_ctas();
   launch_chain(kern, dim3(g.num_items < sms ? g.num_items : sms), dim3(256), smem, st, tmX128, tmXhh, tmG136, g, dW, db);
@@ -404,27 +384,24 @@ int tc_wgrad_x3(const uint16_t* x, const uint16_t* gsrc, float* dW, float* db, i
   return UDH_ENOSUP;
 }
 
-int pad_cast_x3(const float* src, uint16_t* dst, int B, int H, int W, int C, bool grad, cudaStream_t st) {
+int pad_cast_x3(const float* src, uint16_t* dst, int B, int H, int W, int C, cudaStream_t st) {
   const size_t total = (size_t)B * H * W * (C / 4);
-  if (grad) launch_chain(pad_cast_x3_kernel<kGrad>, dim3(grid1d((total + 255) / 256, 148 * 32)), dim3(256), 0, st, src, dst, B, H, W, C);
-  else launch_chain(pad_cast_x3_kernel<kFwd>, dim3(grid1d((total + 255) / 256, 148 * 32)), dim3(256), 0, st, src, dst, B, H, W, C);
+  launch_chain(pad_cast_x3_kernel, dim3(grid1d((total + 255) / 256, 148 * 32)), dim3(256), 0, st, src, dst, B, H, W, C);
   return check_launch("pad_cast_x3");
 }
-int unpad_cast_x3(const uint16_t* src, float* dst, int B, int H, int W, int C, bool grad, cudaStream_t st) {
+int unpad_cast_x3(const uint16_t* src, float* dst, int B, int H, int W, int C, cudaStream_t st) {
   const size_t total = (size_t)B * H * W * (C / 4);
-  if (grad) unpad_cast_x3_kernel<kGrad><<<grid1d((total + 255) / 256, 148 * 32), 256, 0, st>>>(src, dst, B, H, W, C);
-  else unpad_cast_x3_kernel<kFwd><<<grid1d((total + 255) / 256, 148 * 32), 256, 0, st>>>(src, dst, B, H, W, C);
+  unpad_cast_x3_kernel<<<grid1d((total + 255) / 256, 148 * 32), 256, 0, st>>>(src, dst, B, H, W, C);
   return check_launch("unpad_cast_x3");
 }
-int cast_x3(const float* src, uint16_t* dst, size_t rows, int cols, bool grad, cudaStream_t st) {
+int cast_x3(const float* src, uint16_t* dst, size_t rows, int cols, cudaStream_t st) {
   const size_t total = rows * (cols / 4);
-  if (grad) launch_chain(cast_x3_kernel<kGrad>, dim3(grid1d((total + 255) / 256, 148 * 16)), dim3(256), 0, st, src, dst, rows, cols);
-  else launch_chain(cast_x3_kernel<kFwd>, dim3(grid1d((total + 255) / 256, 148 * 16)), dim3(256), 0, st, src, dst, rows, cols);
+  launch_chain(cast_x3_kernel, dim3(grid1d((total + 255) / 256, 148 * 16)), dim3(256), 0, st, src, dst, rows, cols);
   return check_launch("cast_x3");
 }
 int pool_fwd_x3(const uint16_t* in, uint16_t* out, uint32_t* codes, int B, int H, int W, int C, cudaStream_t st) {
   const size_t total = (size_t)B * (H / 2) * (W / 2) * (C / 8);
-  launch_chain(pool_fwd_x3_kernel<kFwd>, dim3(grid1d((total + 255) / 256, 148 * 32)), dim3(256), 0, st, in, out, codes, B, H, W, C);
+  launch_chain(pool_fwd_x3_kernel, dim3(grid1d((total + 255) / 256, 148 * 32)), dim3(256), 0, st, in, out, codes, B, H, W, C);
   return check_launch("pool_fwd_x3");
 }
 int pool_bwd_x3(const uint32_t* codes, const uint16_t* gout, uint16_t* gin, int B, int H, int W, int C, cudaStream_t st) {
@@ -443,7 +420,7 @@ int conv1_x3_fwd(const float* I1, const float* I2, const float* w, const float* 
   uint32_t box[2] = {64, 32};
   TRY(tc::make_tmap_bf16(&tmOut, out_limbs, 2, dims, str, box));
   const size_t smem = 1024 + 2 * 16384 + 16384 + 16384 + 256;
-  auto kern = tc::conv1_x3_fwd_kernel<kFwd>;
+  auto kern = tc::conv1_x3_fwd_kernel;
   UDH_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int want = tc::kConv1X3CtasPerSm * persistent_ctas();
   const int grid = g.tiles < want ? g.tiles : want;
@@ -460,7 +437,7 @@ int conv1_x3_wgrad(const float* I1, const float* I2, const uint16_t* G_limbs, fl
   uint32_t box[2] = {64, 128};
   TRY(tc::make_tmap_bf16(&tmG, G_limbs, 2, dims, str, box));
   const size_t smem = 1024 + 2 * 16384 + 4 * 16384 + 256;
-  auto kern = tc::conv1_x3_wgrad_kernel<kFwd, kGrad>;
+  auto kern = tc::conv1_x3_wgrad_kernel;
   UDH_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int want = tc::kConv1X3WgradCtasPerSm * persistent_ctas();
   const int grid = g.tiles < want ? g.tiles : want;
@@ -470,9 +447,9 @@ int conv1_x3_wgrad(const float* I1, const float* I2, const uint16_t* G_limbs, fl
 
 inline uint16_t* U16(char* base, size_t off) { return reinterpret_cast<uint16_t*>(base + off); }
 
-// conv1_2 on row tiles (forward fused with pool1, row-tile dgrad): on by default, UDH_X3_ROWS=0 / udh_debug_x3_set_rows(0)
-// select the generic flattened-tile kernels + the separate pool kernel (tests compare the two)
-int g_x3_rows = [] { const char* e = getenv("UDH_X3_ROWS"); return (e && e[0] == '0') ? 0 : 1; }();
+// conv1_2 on row tiles (forward fused with pool1, row-tile dgrad): on by default, udh_debug_x3_set_rows(0) selects the
+// generic flattened-tile kernels + the separate pool kernel (tests compare the two)
+int g_x3_rows = 1;
 
 }  // namespace
 
@@ -502,15 +479,15 @@ int x3_cnn_fwd_convs(const float* params, const size_t* poff, const float* I1, c
     const int s = P / kConv[i].div;
     if (i == 1 && fuse_pool1) {
       ProfScope ps(PROF_CONV_FWD0 + i, st);
-      TRY((launch_conv_x3_rows<1, kFwd, kFwd, kFwd>(U16(tcw, L.P[0]), U16(tcw, L.wf[1]), params + poff[3], nullptr,
-                                                    reinterpret_cast<uint32_t*>(tcw + L.Px[0]), U16(tcw, L.P[8]), 1, B, s, s, st)));
+      TRY((launch_conv_x3_rows<1>(U16(tcw, L.P[0]), U16(tcw, L.wf[1]), params + poff[3], nullptr,
+                                  reinterpret_cast<uint32_t*>(tcw + L.Px[0]), U16(tcw, L.P[8]), 1, B, s, s, st)));
       continue;
     }
     {
       ProfScope ps(PROF_CONV_FWD0 + i, st);
-      TRY((tc_conv_x3<kFwd, kFwd, kFwd>(U16(tcw, L.P[input_of(i)]), U16(tcw, L.wf[i]), params + poff[2 * i + 1], nullptr,
-                                        (i % 2 == 0) ? reinterpret_cast<uint32_t*>(tcw + L.Mb[i]) : nullptr, U16(tcw, L.P[i]),
-                                        i == 7 ? at<float>(ws, act_off[7]) : nullptr, 1, B, s, s, kConv[i].cin, kConv[i].cout, st)));
+      TRY(tc_conv_x3(U16(tcw, L.P[input_of(i)]), U16(tcw, L.wf[i]), params + poff[2 * i + 1], nullptr,
+                     (i % 2 == 0) ? reinterpret_cast<uint32_t*>(tcw + L.Mb[i]) : nullptr, U16(tcw, L.P[i]),
+                     i == 7 ? at<float>(ws, act_off[7]) : nullptr, 1, B, s, s, kConv[i].cin, kConv[i].cout, st));
     }
     if (i == 1 || i == 3 || i == 5) {
       ProfScope ps(PROF_POOL_FWD, st);
@@ -527,15 +504,14 @@ int x3_cnn_bwd_convs(const float* params, const size_t* poff, const float* I1, c
   char* tcw = at<char>(ws, tc_off);
   {
     ProfScope ps(PROF_TC_PREP, st);        // (the mirrored weight packs were made by the forward of this step)
-    TRY(pad_cast_x3(gA, U16(tcw, L.G[7]), B, P / 8, P / 8, 128, true, st));
+    TRY(pad_cast_x3(gA, U16(tcw, L.G[7]), B, P / 8, P / 8, 128, st));
   }
-  const int reserve_all = g_sm_reserve;
-  struct RestoreReserve { int v; ~RestoreReserve() { g_sm_reserve = v; } } restore_reserve{reserve_all};
+  struct RestoreReserve { ~RestoreReserve() { g_sm_reserve = 0; } } restore_reserve;   // outside the conv backward every SM is used
   for (int i = 7; i >= 0; --i) {
     TRY(bwd_marker_record(i, st));
     const int s = P / kConv[i].div;
     const int cin = kConv[i].cin, cout = kConv[i].cout;
-    g_sm_reserve = bwd_sm_reserve(i, reserve_all);   // see udh_set_sm_reserve_top / udh_set_sm_reserve_marker
+    g_sm_reserve = bwd_sm_reserve(i);   // see udh_set_sm_reserve_top
     {
       ProfScope ps(PROF_CONV_WGRAD0 + i, st);
       if (i == 0) TRY(conv1_x3_wgrad(I1, I2, U16(tcw, L.G[0]), grads + poff[0], grads + poff[1], B, s, s, st));
@@ -546,16 +522,16 @@ int x3_cnn_bwd_convs(const float* params, const size_t* poff, const float* I1, c
     const int below = input_of(i);
     if (i == 1 && g_x3_rows && P == 128) {
       ProfScope ps(PROF_CONV_DGRAD0 + i, st);                 // conv1_2 dgrad on row tiles, ReLU mask of conv1_1 fused
-      TRY((launch_conv_x3_rows<2, kGrad, kGrad, kGrad>(U16(tcw, L.G[1]), U16(tcw, L.wd[1]), nullptr, reinterpret_cast<const uint32_t*>(tcw + L.Mb[0]),
-                                                       nullptr, U16(tcw, L.G[0]), 0, B, s, s, st)));
+      TRY((launch_conv_x3_rows<2>(U16(tcw, L.G[1]), U16(tcw, L.wd[1]), nullptr, reinterpret_cast<const uint32_t*>(tcw + L.Mb[0]),
+                                  nullptr, U16(tcw, L.G[0]), 0, B, s, s, st)));
       continue;
     }
     {
       ProfScope ps(PROF_CONV_DGRAD0 + i, st);
       // dgrad = conv of G[i] with the mirrored kernel; ReLU mask of the layer below fused unless a pool sits between
-      TRY((tc_conv_x3<kGrad, kGrad, kGrad>(U16(tcw, L.G[i]), U16(tcw, L.wd[i]), nullptr,
-                                           below_is_pool ? nullptr : reinterpret_cast<const uint32_t*>(tcw + L.Mb[below]), nullptr,
-                                           U16(tcw, L.G[below]), nullptr, 0, B, s, s, cout, cin, st)));
+      TRY(tc_conv_x3(U16(tcw, L.G[i]), U16(tcw, L.wd[i]), nullptr,
+                     below_is_pool ? nullptr : reinterpret_cast<const uint32_t*>(tcw + L.Mb[below]), nullptr,
+                     U16(tcw, L.G[below]), nullptr, 0, B, s, s, cout, cin, st));
     }
     if (below_is_pool) {
       ProfScope ps(PROF_POOL_BWD, st);
@@ -575,7 +551,7 @@ int x3_materialize_acts(void* ws, const size_t* act_off, size_t tc_off, int B, i
     if (i == 1 && P == 128 && g_x3_rows) continue;           // conv1_2 is fused with pool1: its full-resolution output is never stored
     const int s = i < 8 ? P / kConv[i].div : P >> (i - 7);
     const int c = i < 8 ? kConv[i].cout : (i == 10 ? 128 : 64);
-    TRY(unpad_cast_x3(U16(tcw, L.P[i]), at<float>(ws, act_off[i]), B, s, s, c, false, st));
+    TRY(unpad_cast_x3(U16(tcw, L.P[i]), at<float>(ws, act_off[i]), B, s, s, c, st));
   }
   return UDH_OK;
 }
@@ -600,17 +576,17 @@ int x3_fc1_fwd(const float* x, const float* w, float* acc, void* ws, size_t tc_o
   const size_t feat = (size_t)(P / 8) * (P / 8) * 128;
   uint16_t* xb = U16(tcw, L.fc_x);
   uint16_t* wb = U16(tcw, L.fc_w);
-  TRY(cast_x3(x, xb, (size_t)B, (int)feat, false, st));
+  TRY(cast_x3(x, xb, (size_t)B, (int)feat, st));
   if (!w_mirror_current) {
     const size_t n4 = feat * 1024 / 4;
-    launch_chain(cast_planes_x3_kernel<kFwd>, dim3(grid1d((n4 + 255) / 256, 148 * 16)), dim3(256), 0, st, w, wb, wb + feat * 1024, n4);
+    launch_chain(cast_planes_x3_kernel, dim3(grid1d((n4 + 255) / 256, 148 * 16)), dim3(256), 0, st, w, wb, wb + feat * 1024, n4);
     TRY(check_launch("cast_planes_x3"));
   }
   const int kb = 3 * (int)(feat / 64);
   int splits = 32;
   while (kb % splits) splits >>= 1;
   tc::GemmSegments seg = {3, {(int)feat, 0, 0}, {0, 0, 0}, {0, 0, (int)feat}, {0, 0, 0}};
-  return tc::launch_gemm<false, true, true, kFwd, kFwd>(xb, 2 * feat, (uint64_t)B, wb, 1024, 2 * feat, acc, 1024, B, 1024, (int)feat, splits, &seg, st);
+  return tc::launch_gemm<false, true, true>(xb, 2 * feat, (uint64_t)B, wb, 1024, 2 * feat, acc, 1024, B, 1024, (int)feat, splits, &seg, st);
 }
 
 // fc1 backward: dW[F,1024] = x^T . dy (stored), dx[B,F] = dy . W^T, from the limb copies of x and W made by the forward
@@ -621,13 +597,13 @@ int x3_fc1_bwd(const float* dy, float* dW, float* dx, void* ws, size_t tc_off, i
   uint16_t* xb = U16(tcw, L.fc_x);
   uint16_t* wb = U16(tcw, L.fc_w);
   uint16_t* dyb = U16(tcw, L.fc_dy);
-  TRY(cast_x3(dy, dyb, (size_t)B, 1024, true, st));
+  TRY(cast_x3(dy, dyb, (size_t)B, 1024, st));
   // dW = x^T . dy: A = x limbs read MN-major (m = feature), B = dy limbs MN-major (n = output); K = batch
   tc::GemmSegments sw = {3, {0, 0, 0}, {(int)feat, 0, 0}, {0, 0, 0}, {0, 0, 1024}};
-  TRY((tc::launch_gemm<true, true, false, kFwd, kGrad>(xb, 2 * feat, (uint64_t)B, dyb, 2048, (uint64_t)B, dW, 1024, (int)feat, 1024, B, 1, &sw, st)));
+  TRY((tc::launch_gemm<true, true, false>(xb, 2 * feat, (uint64_t)B, dyb, 2048, (uint64_t)B, dW, 1024, (int)feat, 1024, B, 1, &sw, st)));
   // dx = dy . W^T: A = dy limbs K-major, B = W limbs as [n = feature][k = 1024] K-major (W_lo rows start at row F)
   tc::GemmSegments sx = {3, {1024, 0, 0}, {0, 0, 0}, {0, 0, 0}, {0, 0, (int)feat}};
-  return tc::launch_gemm<false, false, false, kGrad, kFwd>(dyb, 2048, (uint64_t)B, wb, 1024, 2 * feat, dx, (int64_t)feat, B, (int)feat, 1024, 1, &sx, st);
+  return tc::launch_gemm<false, false, false>(dyb, 2048, (uint64_t)B, wb, 1024, 2 * feat, dx, (int64_t)feat, B, (int)feat, 1024, 1, &sx, st);
 }
 
 // ---- debug / test entries: one x3 layer on fp32 NHWC tensors (splits into limbs internally) --------------------------
@@ -646,7 +622,7 @@ __global__ void pack_one_x3_kernel(const float* __restrict__ w, uint16_t* __rest
     const int kc = cb * 64 + k;
     const float v = dgrad ? w[((size_t)(8 - tap) * Cin + n) * Cout + kc] : w[((size_t)tap * Cin + kc) * Cout + n];
     uint16_t hi, lo;
-    if (dgrad) split1<kGrad>(v, hi, lo); else split1<kFwd>(v, hi, lo);
+    split1(v, hi, lo);
     const size_t blk = (size_t)(tap * CBk + cb) * 2;
     dst[(blk * N + n) * 64 + k] = hi;
     dst[((blk + 1) * N + n) * 64 + k] = lo;
@@ -661,12 +637,11 @@ int x3_debug_conv(const float* x, const float* w, const float* bias, float* out,
   uint16_t* op = reinterpret_cast<uint16_t*>(s + al256((size_t)B * (H + 2) * (W + 2) * kin * 4));
   uint16_t* wp = reinterpret_cast<uint16_t*>(s + al256((size_t)B * (H + 2) * (W + 2) * kin * 4) + al256((size_t)B * (H + 2) * (W + 2) * kout * 4));
   UDH_CUDA(cudaMemsetAsync(scratch, 0, x3_debug_scratch_bytes(B, H, W, cin, cout), st));
-  TRY(pad_cast_x3(x, xp, B, H, W, kin, dgrad != 0, st));
+  TRY(pad_cast_x3(x, xp, B, H, W, kin, st));
   pack_one_x3_kernel<<<(9 * cin * cout + 255) / 256, 256, 0, st>>>(w, wp, cin, cout, dgrad);
   TRY(check_launch("pack_one_x3"));
-  if (dgrad) TRY((tc_conv_x3<kGrad, kGrad, kGrad>(xp, wp, bias, nullptr, nullptr, op, nullptr, relu, B, H, W, kin, kout, st)));
-  else TRY((tc_conv_x3<kFwd, kFwd, kFwd>(xp, wp, bias, nullptr, nullptr, op, nullptr, relu, B, H, W, kin, kout, st)));
-  return unpad_cast_x3(op, out, B, H, W, kout, dgrad != 0, st);
+  TRY(tc_conv_x3(xp, wp, bias, nullptr, nullptr, op, nullptr, relu, B, H, W, kin, kout, st));
+  return unpad_cast_x3(op, out, B, H, W, kout, st);
 }
 
 int x3_debug_wgrad(const float* x, const float* gsrc, float* dW, float* db, void* scratch, int B, int H, int W, int cin, int cout, cudaStream_t st) {
@@ -674,8 +649,8 @@ int x3_debug_wgrad(const float* x, const float* gsrc, float* dW, float* db, void
   uint16_t* xp = reinterpret_cast<uint16_t*>(s);
   uint16_t* gp = reinterpret_cast<uint16_t*>(s + al256((size_t)B * (H + 2) * (W + 2) * cin * 4));
   UDH_CUDA(cudaMemsetAsync(scratch, 0, x3_debug_scratch_bytes(B, H, W, cin, cout), st));
-  TRY(pad_cast_x3(x, xp, B, H, W, cin, false, st));
-  TRY(pad_cast_x3(gsrc, gp, B, H, W, cout, true, st));
+  TRY(pad_cast_x3(x, xp, B, H, W, cin, st));
+  TRY(pad_cast_x3(gsrc, gp, B, H, W, cout, st));
   return tc_wgrad_x3(xp, gp, dW, db, B, H, W, cin, cout, st);
 }
 
@@ -688,11 +663,11 @@ int x3_debug_conv1(const float* I1, const float* I2, const float* w, const float
   UDH_CUDA(cudaMemsetAsync(scratch, 0, sbytes, st));
   if (out) {
     TRY(conv1_x3_fwd(I1, I2, w, bias, op, nullptr, B, H, W, st));
-    TRY(unpad_cast_x3(op, out, B, H, W, 64, false, st));
+    TRY(unpad_cast_x3(op, out, B, H, W, 64, st));
   }
   if (g) {
     UDH_CUDA(cudaMemsetAsync(scratch, 0, sbytes, st));
-    TRY(pad_cast_x3(g, op, B, H, W, 64, true, st));
+    TRY(pad_cast_x3(g, op, B, H, W, 64, st));
     TRY(conv1_x3_wgrad(I1, I2, op, dW, db, B, H, W, st));
   }
   return UDH_OK;

@@ -42,7 +42,8 @@ struct ConvX3Smem {
 // STAGES > 0: the ring depth is a compile-time constant that divides the stages of an item, so every item starts at ring
 // slot 0 and the MMA issue loop is fully unrolled with static slots, parities and tap offsets (ncu of the dynamic loop:
 // the weights were never late, but ~90 bookkeeping instructions of the single issuing lane between two groups of MMAs let
-// the tensor pipe drain — 54 % active where the issue mix allows 84 %).  STAGES == 0: runtime ring (any depth).
+// the tensor pipe drain — 54 % active where the issue mix allows 84 %).  STAGES == 0: runtime ring (any depth).  The WIDE
+// kernels take the static ring and the other layers the runtime ring, so WIDE == (STAGES > 0).
 // ROWS (W == 128 images, 64 -> 64 channels, T == 2: conv1_2).  An item is the interior of two consecutive image rows
 // (2y, 2y+1): tile t starts at the first interior position of row 2y + t, i.e. the tiles are Wp (not 128) positions apart in
 // the same staged rows, no border position is computed, and the epilogue thread of column x holds both rows of that column.
@@ -50,7 +51,7 @@ struct ConvX3Smem {
 //              exchange), then the POOLED two-limb stream and the 3-bit routing codes of the max-pool backward are written; the
 //              full-resolution activation (554 MB in this mode) is never written or re-read;
 //   ROWS == 2: the ordinary epilogue (bias / ReLU-backward mask / limb split / TMA store) on row tiles (the dgrad).
-template <int N_OUT, int CB, int T, int FMT_A, int FMT_W, int FMT_O, bool WIDE = false, int STAGES = 0, int ROWS = 0>
+template <int N_OUT, int CB, int T, bool WIDE = false, int STAGES = 0, int ROWS = 0>
 __global__ void __launch_bounds__(384, 1)
 tc_conv_x3_kernel(const __grid_constant__ CUtensorMap tmA128, const __grid_constant__ CUtensorMap tmAhh,
                   const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CUtensorMap tmOut, const ConvGeom g,
@@ -62,7 +63,8 @@ tc_conv_x3_kernel(const __grid_constant__ CUtensorMap tmA128, const __grid_const
   uint8_t* sA = base;                                             // [2 limbs][CB][abuf_rows][128]
   uint8_t* sW = base + (size_t)2 * CB * abuf_bytes;               // [stages][N_OUT][128]
   static_assert(!WIDE || (N_OUT == 64 && T <= 2), "WIDE: 64 output channels, two accumulators per tile");
-  static_assert(ROWS == 0 || (WIDE && STAGES > 0 && CB == 1 && T == 2), "row tiles: the WIDE static-ring instance with two tiles");
+  static_assert(WIDE == (STAGES > 0), "WIDE kernels use the static ring, the others the runtime ring");
+  static_assert(ROWS == 0 || (WIDE && CB == 1 && T == 2), "row tiles: the WIDE instance with two tiles");
   constexpr bool POOL = ROWS == 1;
   // first position of an item and distance between its tiles (in positions)
   auto item_q0 = [&](int item) { return ROWS ? ((item / (g.H >> 1)) * g.Hp + 2 * (item % (g.H >> 1)) + 1) * g.Wp + 1 : item * T * 128; };
@@ -148,8 +150,8 @@ tc_conv_x3_kernel(const __grid_constant__ CUtensorMap tmA128, const __grid_const
   } else if (warp == 1) {
     // ===================================== MMA issuer =====================================
     // The whole warp stays converged (descriptors live in uniform registers); one elected lane issues.
-    constexpr uint32_t idesc = make_idesc_f16kind(128, N_OUT, 0, 0, FMT_A, FMT_W);
-    constexpr uint32_t idesc_wide = make_idesc_f16kind(128, 2 * N_OUT, 0, 0, FMT_A, FMT_W);
+    constexpr uint32_t idesc = make_idesc_bf16(128, N_OUT, 0, 0);
+    constexpr uint32_t idesc_wide = make_idesc_bf16(128, 2 * N_OUT, 0, 0);
     const uint32_t a_addr0 = smem_u32(sA), w_addr0 = smem_u32(sW);
     // ring position as a running (stage, parity) pair and taps as running (ky, kx) counters: the issue loop of this single
     // warp is the serial resource of the kernel, so it carries no integer division and no per-block address rebuild
@@ -157,7 +159,7 @@ tc_conv_x3_kernel(const __grid_constant__ CUtensorMap tmA128, const __grid_const
     const uint32_t w_stage_units = (uint32_t)kStageBytes >> 4;
     const uint32_t w_lo0 = desc_lo(w_addr0, 16);
     if constexpr (STAGES > 0) {
-      constexpr int kHiStages = (WIDE ? 9 : 18) * CB, kSPI = kHiStages + 9 * CB;      // ring stages of phase HI / of an item
+      constexpr int kHiStages = 9 * CB, kSPI = kHiStages + 9 * CB;                   // ring stages of phase HI / of an item
       static_assert(kSPI % STAGES == 0, "the static ring depth must divide the stages of an item");
       constexpr int kPasses = kSPI / STAGES;
       const uint32_t cb_units = (uint32_t)abuf_bytes >> 4;
@@ -177,8 +179,7 @@ tc_conv_x3_kernel(const __grid_constant__ CUtensorMap tmA128, const __grid_const
           for (int j = 0; j < kSPI; ++j) {
             const bool hi = j < kHiStages;
             const int jj = hi ? j : j - kHiStages;
-            const int kb = (hi && !WIDE) ? (jj >> 1) : jj;        // (tap, cb) index
-            const int tap = kb / CB, cb = kb - tap * CB;
+            const int tap = jj / CB, cb = jj - tap * CB;
             const int ky = tap / 3, kx = tap - ky * 3;
             const int s = j % STAGES;
             if (j == kHiStages) {                                 // phase HI done: release the hi rows, take the lo rows
@@ -190,7 +191,7 @@ tc_conv_x3_kernel(const __grid_constant__ CUtensorMap tmA128, const __grid_const
             tc_fence_after();
             const uint32_t a_lo = (hi ? a_hi0 : a_lo0) + (uint32_t)ky * wp8 + (uint32_t)(kx * 8) + (uint32_t)cb * cb_units;
             const uint32_t w_lo = w_lo0 + (uint32_t)s * w_stage_units;
-            const uint32_t id = (WIDE && hi) ? idesc_wide : idesc;
+            const uint32_t id = hi ? idesc_wide : idesc;
 #pragma unroll
             for (int t = 0; t < T; ++t) {
 #pragma unroll
@@ -230,17 +231,16 @@ tc_conv_x3_kernel(const __grid_constant__ CUtensorMap tmA128, const __grid_const
               for (int cb = 0; cb < CB; ++cb) {
 #pragma unroll
                 for (int wl = 0; wl < 2; ++wl) {
-                  if (wl == 1 && (ph == 1 || WIDE)) continue;     // phase LO multiplies with W_hi only; WIDE: one [hi | lo] stage
+                  if (wl == 1 && ph == 1) continue;               // phase LO multiplies with W_hi only
                   mbar_wait(&w_full[ws], wpar);
                   tc_fence_after();
                   const uint32_t a_lo = a_tap + (uint32_t)cb * cb_units;
                   const uint32_t w_lo = w_lo0 + ws * w_stage_units;
-                  const uint32_t id = (WIDE && ph == 0) ? idesc_wide : idesc;
 #pragma unroll
                   for (int t = 0; t < T; ++t) {
 #pragma unroll
                     for (int k = 0; k < 4; ++k)     // +1024 sixteen-byte units per tile, +2 per 32-byte k-step
-                      umma_bf16(d0 + (uint32_t)(t * kTileCols), desc_from_lo(a_lo + t * 1024 + k * 2), desc_from_lo(w_lo + k * 2), id,
+                      umma_bf16(d0 + (uint32_t)(t * kTileCols), desc_from_lo(a_lo + t * 1024 + k * 2), desc_from_lo(w_lo + k * 2), idesc,
                                 (first | (uint32_t)(k > 0)) ? 1u : 0u);
                   }
                   umma_commit(&w_empty[ws]);
@@ -257,7 +257,7 @@ tc_conv_x3_kernel(const __grid_constant__ CUtensorMap tmA128, const __grid_const
       __syncwarp();
       // the elected lane advanced its private copy of the ring position: every lane recomputes it (once per item)
       {
-        constexpr uint32_t kSPI = (uint32_t)((WIDE ? 18 : 27) * CB);
+        constexpr uint32_t kSPI = (uint32_t)(27 * CB);
         const uint32_t tot = ws0 + kSPI;
         ws = tot % (uint32_t)stages;
         wpar = wpar0 ^ ((tot / (uint32_t)stages) & 1u);
@@ -317,7 +317,7 @@ tc_conv_x3_kernel(const __grid_constant__ CUtensorMap tmA128, const __grid_const
         // both lanes of a pair hold the pooled pixel: the even lane stores channels 0-15 of this chunk, the odd 16-31
         uint32_t ph_[8], pl_[8];
 #pragma unroll
-        for (int h = 0; h < 8; ++h) split2<FMT_O>(odd ? m[16 + 2 * h] : m[2 * h], odd ? m[17 + 2 * h] : m[2 * h + 1], ph_[h], pl_[h]);
+        for (int h = 0; h < 8; ++h) split2(odd ? m[16 + 2 * h] : m[2 * h], odd ? m[17 + 2 * h] : m[2 * h + 1], ph_[h], pl_[h]);
         uint4* oh = reinterpret_cast<uint4*>(prow + c * 32 + odd * 16);
         oh[0] = make_uint4(ph_[0], ph_[1], ph_[2], ph_[3]); oh[1] = make_uint4(ph_[4], ph_[5], ph_[6], ph_[7]);
         uint4* ol = reinterpret_cast<uint4*>(prow + 64 + c * 32 + odd * 16);
@@ -400,7 +400,7 @@ tc_conv_x3_kernel(const __grid_constant__ CUtensorMap tmA128, const __grid_const
           uint32_t hi[16], lo[16];
 #pragma unroll
           for (int j = 0; j < 16; ++j) {
-            if (valid) split2<FMT_O>(v[2 * j], v[2 * j + 1], hi[j], lo[j]);
+            if (valid) split2(v[2 * j], v[2 * j + 1], hi[j], lo[j]);
             else { hi[j] = 0u; lo[j] = 0u; }                       // border / out-of-range positions store zeros
           }
 #pragma unroll

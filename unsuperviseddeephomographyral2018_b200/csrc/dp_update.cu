@@ -12,7 +12,6 @@
 // two symmetric-memory barriers enqueued by the host around this launch (engine.py); the kernel itself never waits on a peer.
 #include "common.cuh"
 #include "tc_common.cuh"
-#include "x3_config.cuh"
 
 namespace udh {
 
@@ -32,8 +31,8 @@ __device__ __forceinline__ void mm_st(uint2* mc, const uint2& v) {
 }
 
 constexpr int kDpUnroll = 4;   // multicast loads in flight per thread (a switch round trip is a few microseconds)
-// The kernel runs on a handful of SMs of its own (the conv kernels next to it own theirs outright, udh_set_sm_reserve_marker):
-// large CTAs with every load of an iteration issued up front, so that those few SMs keep enough bytes in flight.
+// The kernel takes turns on the SMs with the conv kernels next to it (a conv CTA owns its SM outright): large CTAs with every
+// load of an iteration issued up front, so that each SM it gets keeps enough bytes in flight.
 constexpr int kDpThreads = 512;
 
 // LIMBS: 0 = no mirror (fp32 mode), 1 = one bf16 plane, 2 = hi + lo planes (p = hi + lo)
@@ -69,8 +68,8 @@ __global__ void __launch_bounds__(kDpThreads) dp_shard_update_kernel(const float
         mm_st(mc_p + i, P);
         if (LIMBS == 2) {
           uint2 h, l;
-          tc::split2<kX3Fwd>(P.x, P.y, h.x, l.x);
-          tc::split2<kX3Fwd>(P.z, P.w, h.y, l.y);
+          tc::split2(P.x, P.y, h.x, l.x);
+          tc::split2(P.z, P.w, h.y, l.y);
           mm_st(mc_hi + (i - mb4), h);
           mm_st(mc_lo + (i - mb4), l);
         } else if (LIMBS == 1) {

@@ -32,7 +32,7 @@ constexpr int kGemmEpiBytes = 2 * 4 * 32 * 128;  // TMA-store staging of the non
 
 // ATOMIC: split-K partial tiles are added with 16-byte vector reductions.  Otherwise the tile is stored through a swizzled
 // shared-memory staging block and TMA (full 128-byte lines; rows / columns beyond M / N are clipped by the tensor map).
-template <bool A_MN, bool B_MN, bool ATOMIC, int FMT_A = kFmtBF16, int FMT_B = kFmtBF16>
+template <bool A_MN, bool B_MN, bool ATOMIC>
 __global__ void __launch_bounds__(256, 1)
 tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const __grid_constant__ CUtensorMap tmC,
                const GemmGeom g, float* __restrict__ C) {
@@ -100,7 +100,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     }
   } else if (warp == 1) {
     // whole warp converged; one elected lane issues
-    constexpr uint32_t idesc = make_idesc_f16kind(128, 256, A_MN ? 1 : 0, B_MN ? 1 : 0, FMT_A, FMT_B);
+    constexpr uint32_t idesc = make_idesc_bf16(128, 256, A_MN ? 1 : 0, B_MN ? 1 : 0);
     uint32_t cnt = 0;
     for (int i = 0; i < my_tiles; ++i) {
       const int b = i & 1;
@@ -184,7 +184,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 // seg (nullable): offsets of the contraction segments (see GemmGeom), K is the length of ONE segment.
 struct GemmSegments { int n; int a_koff[3], a_moff[3], b_koff[3], b_noff[3]; };
 
-template <bool A_MN, bool B_MN, bool ATOMIC, int FMT_A = kFmtBF16, int FMT_B = kFmtBF16>
+template <bool A_MN, bool B_MN, bool ATOMIC>
 inline int launch_gemm(const void* A, uint64_t a_inner, uint64_t a_outer, const void* Bm, uint64_t b_inner, uint64_t b_outer,
                        float* C, int64_t ldc, int M, int N, int K, int k_splits, const GemmSegments* seg, cudaStream_t st) {
   GemmGeom g;
@@ -216,7 +216,7 @@ inline int launch_gemm(const void* A, uint64_t a_inner, uint64_t a_outer, const 
   rc = make_tmap(&tmC, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, C, 2, dC, sC, boxC);
   if (rc != UDH_OK) return rc;
   const size_t smem = 1024 + (size_t)kGemmStages * kGemmStageBytes + (ATOMIC ? 0 : kGemmEpiBytes) + 256;
-  auto kern = tc_gemm_kernel<A_MN, B_MN, ATOMIC, FMT_A, FMT_B>;
+  auto kern = tc_gemm_kernel<A_MN, B_MN, ATOMIC>;
   UDH_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int sms = persistent_ctas();
   const int tiles = g.m_tiles * g.n_tiles * g.k_splits;

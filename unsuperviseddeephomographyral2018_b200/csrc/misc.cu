@@ -3,7 +3,7 @@
 #include <string.h>
 
 #include "common.cuh"
-#include "x3_config.cuh"
+#include "tc_common.cuh"
 
 namespace udh {
 
@@ -20,10 +20,8 @@ unsigned long long g_launches = 0;
 int g_sm_reserve = 0;
 int g_sm_reserve_top = 0;
 int g_bwd_marker_layer = -1;   // udh_set_bwd_marker
-int g_sm_reserve_marker = 0;    // udh_set_sm_reserve_marker
 static cudaEvent_t g_bwd_marker_ev = nullptr;
 static bool g_bwd_marker_recorded = false;
-int g_adam_grid = 0;        // udh_set_adam_grid: CTAs of the next Adam launches (0 = fill the device)
 
 namespace {
 const char* kTagNames[PROF_NUM_TAGS] = {
@@ -118,8 +116,8 @@ __global__ void __launch_bounds__(256) adam_kernel(float4* __restrict__ p, float
     if (in_mirror) {
       if (mirror_lo) {             // two-limb mirror (UDH_NUMERIC_BF16X3): p = hi + lo
         uint2 h, l;
-        tc::split2<kX3Fwd>(pv.x, pv.y, h.x, l.x);
-        tc::split2<kX3Fwd>(pv.z, pv.w, h.y, l.y);
+        tc::split2(pv.x, pv.y, h.x, l.x);
+        tc::split2(pv.z, pv.w, h.y, l.y);
         mirror[i - mb4] = h;
         mirror_lo[i - mb4] = l;
       } else {
@@ -147,12 +145,6 @@ extern "C" int udh_device_available(void) {
 
 extern "C" unsigned long long udh_launch_count(void) { return udh::g_launches; }
 
-extern "C" int udh_set_sm_reserve(int n) {
-  UDH_REQUIRE(n >= 0 && n < 128, "udh_set_sm_reserve: bad value %d", n);
-  udh::g_sm_reserve = n;
-  return UDH_OK;
-}
-
 namespace udh {
 int bwd_marker_record(int layer, cudaStream_t st) {
   if (layer != g_bwd_marker_layer) return UDH_OK;
@@ -169,21 +161,9 @@ extern "C" int udh_set_bwd_marker(int layer) {
   return UDH_OK;
 }
 
-extern "C" int udh_set_sm_reserve_marker(int n) {
-  UDH_REQUIRE(n >= 0 && n < 128, "udh_set_sm_reserve_marker: bad value %d", n);
-  udh::g_sm_reserve_marker = n;
-  return UDH_OK;
-}
-
 extern "C" int udh_bwd_marker_wait(void* stream) {
   if (!udh::g_bwd_marker_recorded) return UDH_OK;      // nothing recorded yet: no dependency to add
   UDH_CUDA(cudaStreamWaitEvent(udh::as_stream(stream), udh::g_bwd_marker_ev, 0));
-  return UDH_OK;
-}
-
-extern "C" int udh_set_adam_grid(int blocks) {
-  UDH_REQUIRE(blocks >= 0 && blocks <= 148 * 16, "udh_set_adam_grid: blocks must be in 0..2368");
-  udh::g_adam_grid = blocks;
   return UDH_OK;
 }
 
@@ -256,7 +236,7 @@ extern "C" int udh_adam_step_mirror_ex(float* p, float* g, float* m, float* v, s
   UDH_REQUIRE(((uintptr_t)p | (uintptr_t)g | (uintptr_t)m | (uintptr_t)v) % 16 == 0, "udh_adam_step: buffers must be 16-byte aligned");
   if (n == 0) return UDH_OK;
   const size_t n4 = n / 4;
-  const size_t full = (n4 + 255) / 256, cap = udh::g_adam_grid > 0 ? (size_t)udh::g_adam_grid : (size_t)148 * 16;
+  const size_t full = (n4 + 255) / 256, cap = (size_t)148 * 16;
   const unsigned blocks = (unsigned)(full < cap ? full : cap);
   udh::ProfScope ps(udh::PROF_ADAM, udh::as_stream(stream));
   udh::launch_chain(udh::adam_kernel, dim3(blocks), dim3(256), 0, udh::as_stream(stream), (float4*)p, (float4*)g, (float4*)m, (float4*)v, n4, alpha_t,

@@ -3,7 +3,6 @@
 #pragma once
 #include <cuda.h>
 #include <cuda_bf16.h>
-#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -178,41 +177,23 @@ __host__ __device__ constexpr uint32_t make_idesc_bf16(int M, int N, int a_mn, i
          ((uint32_t)(M >> 4) << 24);
 }
 
-// Same, with the operand formats spelled out: 0 = fp16, 1 = bf16 (kind::f16 takes either format on either side).
-constexpr int kFmtF16 = 0, kFmtBF16 = 1;
-__host__ __device__ constexpr uint32_t make_idesc_f16kind(int M, int N, int a_mn, int b_mn, int a_fmt, int b_fmt) {
-  return (1u << 4) | ((uint32_t)a_fmt << 7) | ((uint32_t)b_fmt << 10) | ((uint32_t)a_mn << 15) | ((uint32_t)b_mn << 16) |
-         ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-
 // ---- two-limb split of fp32 values (UDH_NUMERIC_BF16X3) ------------------------------------------------------------
-// x = hi + lo with hi = round16(x), lo = round16(x - hi) (x - hi is exact in fp32).  The product of two split values is
+// x = hi + lo with hi = bf16(x), lo = bf16(x - hi) (x - hi is exact in fp32).  The product of two split values is
 // evaluated on the tensor pipe as hi*hi + hi*lo + lo*hi with fp32 accumulation; the dropped lo*lo term and the residual
-// of the split are both <= 2^-16 |x y| for bf16 limbs (2^-22 for fp16 limbs).  Two values are packed per 32-bit word.
-template <int FMT>
+// of the split are both <= 2^-16 |x y|.  Two values are packed per 32-bit word.
+// Why bf16 and not fp16 limbs (22 bits instead of 16): kind::f16 MMAs with fp16 on one side and bf16 on the other raise
+// an illegal-instruction error on B200, so both operands of every MMA share a format, and the weight gradient multiplies
+// activations with gradients (1e-8 .. 1e-2), which do not fit fp16's range without per-tensor loss scaling.
 __device__ __forceinline__ void split2(float a, float b, uint32_t& hi, uint32_t& lo) {
-  if (FMT == kFmtBF16) {
-    const __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
-    const __nv_bfloat162 l = __floats2bfloat162_rn(a - __low2float(h), b - __high2float(h));
-    hi = *reinterpret_cast<const uint32_t*>(&h);
-    lo = *reinterpret_cast<const uint32_t*>(&l);
-  } else {
-    const __half2 h = __floats2half2_rn(a, b);
-    const __half2 l = __floats2half2_rn(a - __low2float(h), b - __high2float(h));
-    hi = *reinterpret_cast<const uint32_t*>(&h);
-    lo = *reinterpret_cast<const uint32_t*>(&l);
-  }
+  const __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
+  const __nv_bfloat162 l = __floats2bfloat162_rn(a - __low2float(h), b - __high2float(h));
+  hi = *reinterpret_cast<const uint32_t*>(&h);
+  lo = *reinterpret_cast<const uint32_t*>(&l);
 }
 // value of a packed pair of limbs: (hi.x + lo.x, hi.y + lo.y)
-template <int FMT>
 __device__ __forceinline__ float2 join2(uint32_t hi, uint32_t lo) {
-  if (FMT == kFmtBF16) {
-    const __nv_bfloat162 h = *reinterpret_cast<const __nv_bfloat162*>(&hi), l = *reinterpret_cast<const __nv_bfloat162*>(&lo);
-    return make_float2(__low2float(h) + __low2float(l), __high2float(h) + __high2float(l));
-  } else {
-    const __half2 h = *reinterpret_cast<const __half2*>(&hi), l = *reinterpret_cast<const __half2*>(&lo);
-    return make_float2(__low2float(h) + __low2float(l), __high2float(h) + __high2float(l));
-  }
+  const __nv_bfloat162 h = *reinterpret_cast<const __nv_bfloat162*>(&hi), l = *reinterpret_cast<const __nv_bfloat162*>(&lo);
+  return make_float2(__low2float(h) + __low2float(l), __high2float(h) + __high2float(l));
 }
 
 // D[tmem] (+)= A[smem] . B[smem]   (issued by ONE thread)

@@ -21,20 +21,21 @@ namespace tc {
 
 constexpr int kConstBlockBytes = 2048;     // 16 positions x 64 channels x 2 bytes
 
-__device__ __forceinline__ void fill_const_blocks(uint8_t* sOnes, uint8_t* sZeros, uint32_t one_pair) {
+constexpr uint32_t kOnePair = 0x3F803F80u;   // two bf16 1.0 packed in one word
+
+__device__ __forceinline__ void fill_const_blocks(uint8_t* sOnes, uint8_t* sZeros) {
   uint32_t* o = reinterpret_cast<uint32_t*>(sOnes);
   uint32_t* z = reinterpret_cast<uint32_t*>(sZeros);
-  for (int i = threadIdx.x; i < kConstBlockBytes / 4; i += blockDim.x) { o[i] = one_pair; z[i] = 0u; }
+  for (int i = threadIdx.x; i < kConstBlockBytes / 4; i += blockDim.x) { o[i] = kOnePair; z[i] = 0u; }
   fence_proxy_async();                                          // generic-proxy writes -> visible to the tensor (async) proxy
 }
-template <int FMT> __host__ __device__ constexpr uint32_t one_pair_bits() { return FMT == kFmtBF16 ? 0x3F803F80u : 0x3C003C00u; }
 
 // buffer indices
 constexpr int kXH = 0, kXL = 1, kGH = 2, kGL = 3;
 
 // ---------------------------------------------------------------------------------------------------------------------
 // generic kernel: N_OUT = 128; CBX = 1 (64 -> 128: two taps per MMA) or 2 (128 -> 128: one tap per MMA + ones group)
-template <int N_OUT, int CBX, int T, int FMT_X, int FMT_G>
+template <int N_OUT, int CBX, int T>
 __global__ void __launch_bounds__(256, 1)
 tc_wgrad_x3_kernel(const __grid_constant__ CUtensorMap tmX128, const __grid_constant__ CUtensorMap tmXhh,
                    const __grid_constant__ CUtensorMap tmG, const WgradGeom g, float* __restrict__ dW, float* __restrict__ db) {
@@ -63,7 +64,7 @@ tc_wgrad_x3_kernel(const __grid_constant__ CUtensorMap tmX128, const __grid_cons
   const int g_count = g.slice_group[sl + 1] - g_begin;
   constexpr int kTmemCols = 512;
 
-  fill_const_blocks(sOnes, sZeros, one_pair_bits<FMT_X>());
+  fill_const_blocks(sOnes, sZeros);
   if (threadIdx.x == 0) {
     for (int i = 0; i < 4; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
     mbar_init(acc_full, 1);
@@ -111,8 +112,8 @@ tc_wgrad_x3_kernel(const __grid_constant__ CUtensorMap tmX128, const __grid_cons
   } else if (warp == 1) {
     // One elected lane runs the whole MMA role (waits included); the per-group operand geometry (row shift of the first M
     // block, leading-dimension offset to the second one, constant-block mode) does not depend on the item and is tabulated once.
-    constexpr uint32_t idesc = make_idesc_f16kind(128, N_OUT, 1, 1, FMT_X, FMT_G);
-    constexpr uint32_t idesc_ones = make_idesc_f16kind(64, N_OUT, 1, 1, FMT_X, FMT_G);
+    constexpr uint32_t idesc = make_idesc_bf16(128, N_OUT, 1, 1);
+    constexpr uint32_t idesc_ones = make_idesc_bf16(64, N_OUT, 1, 1);
     const uint32_t ones_addr = smem_u32(sOnes), zeros_addr = smem_u32(sZeros);
     if (elect_one()) {
       int goff[4]; uint32_t glbo[4]; int gmode[4];               // mode 0: fixed lbo; 1: second M block = constant rows; 2: ones group (M = 64)
@@ -222,7 +223,7 @@ tc_wgrad_x3_kernel(const __grid_constant__ CUtensorMap tmX128, const __grid_cons
 // ---------------------------------------------------------------------------------------------------------------------
 // 64 -> 64 channel layers: the N = 192 formulation of tc_wgrad64_kernel (B = three row shifts of G, A = two row shifts of X;
 // two MMAs per 16 positions and pass), with the limb passes above.
-template <int T, int FMT_X, int FMT_G>
+template <int T>
 __global__ void __launch_bounds__(256, 1)
 tc_wgrad64_x3_kernel(const __grid_constant__ CUtensorMap tmX128, const __grid_constant__ CUtensorMap tmXhh,
                      const __grid_constant__ CUtensorMap tmG136, const Wgrad64Geom g, float* __restrict__ dW, float* __restrict__ db) {
@@ -244,7 +245,7 @@ tc_wgrad64_x3_kernel(const __grid_constant__ CUtensorMap tmX128, const __grid_co
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   constexpr int kTmemCols = 512;                                // 2 groups x 192 columns
 
-  fill_const_blocks(sOnes, sZeros, one_pair_bits<FMT_X>());
+  fill_const_blocks(sOnes, sZeros);
   if (threadIdx.x == 0) {
     for (int i = 0; i < 4; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
     mbar_init(acc_full, 1);
@@ -286,7 +287,7 @@ tc_wgrad64_x3_kernel(const __grid_constant__ CUtensorMap tmX128, const __grid_co
       }
     }
   } else if (warp == 1) {
-    constexpr uint32_t idesc = make_idesc_f16kind(128, 192, 1, 1, FMT_X, FMT_G);
+    constexpr uint32_t idesc = make_idesc_bf16(128, 192, 1, 1);
     const uint32_t ones_addr = smem_u32(sOnes), zeros_addr = smem_u32(sZeros);
     for (int it = 0; it < my_items; ++it) {
       const uint32_t par = it & 1;

@@ -104,24 +104,16 @@ class HomographyEngine(object):
         self.global_step = 0
         self._mv_sharded = False
         self._mc = self._dp_setup_multicast() if self._symm else None
-        # second stream: Row G of the fully connected slice under the conv backward.  UDH_OVERLAP_UPDATE=1 also moves that
-        # slice's Adam there at N = 1; measured on B200 it gains nothing (whichever conv kernel starts next waits for the
-        # update's CTAs to leave its SMs: profiles/r2_dp_overlap_experiments.md), so it is off by default.
-        self._overlap_update = os.environ.get("UDH_OVERLAP_UPDATE", "0") == "1"
-        self._comm_stream = torch.cuda.Stream(device=self.device) if (world_size > 1 or self._overlap_update) else None
+        # second stream: Row G of the fully connected slice under the conv backward
+        self._comm_stream = torch.cuda.Stream(device=self.device) if world_size > 1 else None
         # SM policy of this engine's steps (library-global knobs, applied at the start of every step).  A conv CTA with 200+ KB
         # of shared memory shares its SM with nothing, so a second stream's kernel and the persistent conv kernels take turns
         # on an SM rather than overlap:
         #   top: the SMs NCCL's allreduce kernel (NCCL_MAX_CTAS) takes next to conv4_x's backward on the NCCL path — those four
         #     launches have <= 2 items per CTA and lose nothing on 116 CTAs;
-        #   marker layer / SMs: where in the conv backward the multicast kernel (or UDH_OVERLAP_UPDATE's Adam) starts, and how
-        #     many SMs the conv kernels from there on leave to it (0: it queues for SMs like any other kernel).
-        side_kernel = self._mc is not None or self._overlap_update
-        sms = int(os.environ.get("UDH_DP_SMS", "0")) if side_kernel else 0
-        self._sm_policy = dict(reserve=int(os.environ.get("UDH_SM_RESERVE", "0")) if world_size > 1 else 0,
-                               top=int(os.environ.get("UDH_SM_RESERVE_TOP", "32")) if (world_size > 1 and self._mc is None) else 0,
-                               marker=int(os.environ.get("UDH_DP_MARKER_LAYER", "3")) if side_kernel else -1, marker_sms=sms)
-        self._side_adam_grid = int(os.environ.get("UDH_SIDE_ADAM_GRID", str(sms * 8 if sms else 296)))
+        #   marker layer: where in the conv backward the multicast kernel starts (it queues for SMs like any other kernel).
+        self._sm_policy = dict(top=int(os.environ.get("NCCL_MAX_CTAS", "32")) if (world_size > 1 and self._mc is None) else 0,
+                               marker=3 if self._mc is not None else -1)
         # static per-step outputs of the one-call step (udh_step_forward_backward): reused every step
         B, Pz, dev = self.B, self.Pz, self.device
         self._sb = dict(h4p=torch.zeros(B, 8, device=dev), H=torch.zeros(B, 3, 3, device=dev), pred=torch.zeros(B, Pz, Pz, 1, device=dev),
@@ -317,7 +309,7 @@ class HomographyEngine(object):
         rank, N = hp.rank, hp.world_size
         lo, hi, per = dp_shard_range(begin, count, rank, N)
         return dict(hp=hp, hg=hg, hw=hw, mc_params=mcs[0], mc_grads=mcs[1], mc_ws=mcs[2], begin=begin, count=count, shard=(lo, hi),
-                    per=per, rank=rank, N=N, grid=int(os.environ.get("UDH_DP_GRID", "0")))
+                    per=per, rank=rank, N=N)
 
     def _dp_sharded_update(self, alpha):
         """fc1's weights: udh_dp_shard_update (switch-side gradient sum, Adam on this rank's shard, new weights and limbs
@@ -332,7 +324,7 @@ class HomographyEngine(object):
             limbs = 2 if self.numeric == _lib.NUMERIC_BF16X3 else 1
         check(lib.udh_dp_shard_update(ctypes.c_void_p(mc["mc_grads"]), self._p(self.params), ctypes.c_void_p(mc["mc_params"]),
                                       self._p(self.adam_m), self._p(self.adam_v), mirror, lo, hi - lo, mb, mcount, limbs, alpha, 0.9, 0.999,
-                                      1e-8, 1.0 / self.world_size, mc["grid"], ops._stream()), "udh_dp_shard_update")
+                                      1e-8, 1.0 / self.world_size, 0, ops._stream()), "udh_dp_shard_update")     # grid 0: the default
         mc["hg"].barrier(channel=1, timeout_ms=30000)                    # every owner's stores have landed in every replica
         self._mv_sharded = True
 
@@ -351,10 +343,8 @@ class HomographyEngine(object):
 
     def _apply_sm_policy(self):
         pol = self._sm_policy
-        check(lib.udh_set_sm_reserve(pol["reserve"]), "udh_set_sm_reserve")
         check(lib.udh_set_sm_reserve_top(pol["top"]), "udh_set_sm_reserve_top")
         check(lib.udh_set_bwd_marker(pol["marker"]), "udh_set_bwd_marker")
-        check(lib.udh_set_sm_reserve_marker(pol["marker_sms"]), "udh_set_sm_reserve_marker")
 
     def _adam(self, lo, hi, alpha):
         """TF-1 Adam on the float range [lo, hi) of the flat buffers (4-float aligned), on the current stream; refreshes the
@@ -426,7 +416,7 @@ class HomographyEngine(object):
         a = self._fill_args(batch, True)
         st = ops._stream()
         self._apply_sm_policy()
-        if self.world_size == 1 and not self._overlap_update:
+        if self.world_size == 1:
             check(lib.udh_step_forward_backward(ctypes.byref(a), _lib.STEP_ALL, st), "udh_step_forward_backward")
             out = self._step_out(batch)
             out["lr"] = self.update()
@@ -456,22 +446,12 @@ class HomographyEngine(object):
             torch.distributed.all_reduce(self.grads[:w0], group=self.pg)
             self._adam(0, w0, alpha)
         else:
-            if self.world_size > 1:
-                with torch.cuda.stream(side):
-                    torch.distributed.all_reduce(self.grads[head], group=self.pg)
+            with torch.cuda.stream(side):
+                torch.distributed.all_reduce(self.grads[head], group=self.pg)
             check(lib.udh_step_forward_backward(ctypes.byref(a), _lib.STEP_CONVS, st), "udh_step_forward_backward(convs)")
-            if self._overlap_update:
-                with torch.cuda.stream(side):
-                    check(lib.udh_bwd_marker_wait(ops._stream()), "udh_bwd_marker_wait")
-                    check(lib.udh_set_adam_grid(self._side_adam_grid), "udh_set_adam_grid")     # co-resident with the conv CTAs (udh.h)
-                    self._adam(head.start, n, alpha)
-                    check(lib.udh_set_adam_grid(0), "udh_set_adam_grid")
-            if self.world_size > 1:
-                torch.distributed.all_reduce(self.grads[convs], group=self.pg)
-            if self._overlap_update:
-                self._adam(0, head.start, alpha)
+            torch.distributed.all_reduce(self.grads[convs], group=self.pg)
         cur.wait_stream(side)
-        if self._mc is None and not self._overlap_update:
+        if self._mc is None:
             self._adam(0, n, alpha)
         if self._mirror is not None:
             self._mirror_current = True
